@@ -20,11 +20,16 @@ re-score of every returned (id, score) pair), `recall` (recall@k against exact s
 `sweep` (full-sweep HBM micro-benchmark, N=1), `encoder` + `c5_encode_plus_search` (BASELINE config 5).
 Extra knobs (development only; the defaults are the BASELINE configuration): --n --nq --nlist --m --nprobe --k
 --no-sweep --no-recall --no-encoder --no-cpu-baseline --e2e-transfer.
+`--steps` / `--warmup` set the timed / untimed passes of every timed block (search arms, sweep, encoder, config 5).
+`--dump-outputs DIR` writes the (ids, scores) of the last timed search step as DIR/*.npy: the queries and corpus come
+from fixed seeds and the index training is reproducible (ReproducibleTrainingOps), so the same arguments give the same
+outputs and two builds can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
 import json
+import math
 import os
 import subprocess
 import sys
@@ -85,7 +90,15 @@ def parse():
     ap.add_argument("--partition", default="list", choices=["list", "vector"],
                     help="static datastore partition across GPUs: whole inverted lists per GPU, or 1/G of every list")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="CPU-baseline time budget")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the ids and scores the last timed "
+                    "search step returned to DIR/ids.npy (float64) and DIR/scores.npy (float32); above 64 MB a fixed "
+                    "seeded sample of query rows is written, with their row numbers in DIR/rows.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.encoder_only):
+        ap.error("--dump-outputs writes the results of the GPU search arm: not with --impl reference or --encoder-only")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -191,11 +204,51 @@ class ClockSampler:
 
 # ----------------------------------------------------------------------------------------------------------
 # index construction (setup; not timed).  Build side = SURVEY §8f-1, through librsb: k-means / PQ training
-# (`train.py` -> rsb_kmeans_* kernels), list assignment by the tensor-core coarse quantizer (`index.assign`),
-# residual PQ encoding and the interleaved list layout (`rsb_add_preassigned`, `rsb_finalize`).
+# (`train.py` with librsb's assignment kernels; member sums in fixed point, see ReproducibleTrainingOps), list
+# assignment by the tensor-core coarse quantizer (`index.assign`), residual PQ encoding and the interleaved list
+# layout (`rsb_add_preassigned`, `rsb_finalize`).
 # While the corpus streams through, the exact top-k of a query sample is accumulated (librsb Flat kernels) as the
 # ground truth of the recall figure -- the 307 GB fp32 corpus never materialises.
 # ----------------------------------------------------------------------------------------------------------
+def fixed_point_sums(x: torch.Tensor, seg: torch.Tensor, k: int, chunk_elems: int = 1 << 26) -> torch.Tensor:
+    """Sums of the rows of x [n, d] per segment id seg [n] in [0, k), as float32 [k, d].  Every value is rounded to a
+    multiple of 2**-s, with s as fine as the bound n * max|x| < 2**62 allows, and added as an int64: integer addition
+    is exact, so the sums do not depend on the order in which the GPU's atomics add the rows."""
+    n, d = x.shape
+    bound = float(x.abs().max()) * n if n else 0.0
+    scale = 2.0 ** (62 - math.ceil(math.log2(bound))) if bound > 0 else 1.0
+    acc = torch.zeros(k, d, dtype=torch.int64, device=x.device)
+    rows = max(1, chunk_elems // d)                       # bounds the float64 / int64 copies of a chunk
+    for i in range(0, n, rows):
+        acc.index_add_(0, seg[i:i + rows], torch.round(x[i:i + rows].double() * scale).long())
+    return (acc.double() / scale).float()
+
+
+class ReproducibleTrainingOps:
+    """The operations `train.kmeans` / `train.train_pq` run, with the assignments from `assign_ops` (librsb's kernels
+    in the bench) and the member sums from fixed_point_sums.  librsb's accumulate kernels add floats atomically in
+    arrival order, so their sums, the trained index and every search result change a little from run to run; with
+    these the same arguments give the same index, and --dump-outputs compares like with like."""
+
+    def __init__(self, assign_ops):
+        self.assign_ops = assign_ops
+
+    def assign_ip(self, x, c):
+        return self.assign_ops.assign_ip(x, c)
+
+    def pq_assign(self, r, cb):
+        return self.assign_ops.pq_assign(r, cb)
+
+    def accumulate(self, x, a, k):
+        return fixed_point_sums(x, a, k), torch.bincount(a, minlength=k).float()
+
+    def pq_accumulate(self, r, codes, M, ksub):
+        n, d = r.shape
+        entry = (codes.long() + torch.arange(M, device=r.device) * ksub).flatten()    # codebook entry of each sub-vector
+        sums = fixed_point_sums(r.reshape(n * M, d // M), entry, M * ksub)
+        return sums.view(M, ksub, d // M), torch.bincount(entry, minlength=M * ksub).float().view(M, ksub)
+
+
 def build_index(args, rank: int, world: int, device, gt_queries=None):
     import retrieval_scaling_b200 as rsb
     from retrieval_scaling_b200 import synth, train
@@ -210,13 +263,14 @@ def build_index(args, rank: int, world: int, device, gt_queries=None):
     cent = torch.empty(args.nlist, args.d, device=device)
     cb = torch.empty(args.m, 256, args.d // args.m, device=device)
     if rank == 0:
+        ops = ReproducibleTrainingOps(train.LibrsbOps())
         ntrain = min(args.n, args.nlist * args.train_per_centroid)
         xt = corpus.train_sample(ntrain)
-        cent.copy_(train.kmeans(xt, args.nlist, niter=10, metric="ip", spherical=True, seed=1234))
+        cent.copy_(train.kmeans(xt, args.nlist, niter=10, metric="ip", spherical=True, seed=1234, ops=ops))
         xs = xt[: 256 * 256]
-        a = train.assign_ip(xs, cent)
-        cb.copy_(train.train_pq(xs - cent[a], args.m, 256, niter=25, seed=1234))
-        del xt, xs, a
+        a = train.assign_ip(xs, cent, ops=ops)
+        cb.copy_(train.train_pq(xs - cent[a], args.m, 256, niter=25, seed=1234, ops=ops))
+        del xt, xs, a, ops
     if world > 1:
         torch.distributed.broadcast(cent, 0)
         torch.distributed.broadcast(cb, 0)
@@ -327,7 +381,7 @@ def recall_block(I_pq: torch.Tensor, gt_I: torch.Tensor, k: int):
                             "accumulated chunk by chunk during the build"}
 
 
-def sweep_microbench(index, args, cent, device, steps=10, warmup=3):
+def sweep_microbench(index, args, cent, device):
     """Full-sweep HBM micro-benchmark (SURVEY §8d): nlist/nprobe queries whose probe sets partition all lists
     exactly once => pair-bytes == unique bytes == the whole code array, nothing is re-read from L2."""
     nprobe = args.nprobe
@@ -342,11 +396,11 @@ def sweep_microbench(index, args, cent, device, steps=10, warmup=3):
     except Exception:
         pass
     ms, nbytes = [], 0
-    for it in range(warmup + steps):
+    for it in range(args.warmup + args.steps):
         index.search_preassigned(q, args.k, lists, dis)
         torch.cuda.synchronize()
         p = index.profile()
-        if it >= warmup:
+        if it >= args.warmup:
             ms.append(p["scan_ms"]); nbytes = p["scan_bytes"]
     t = float(np.mean(ms))
     return {"queries": nq, "scan_ms": t, "bytes": nbytes, "gbs": nbytes / t / 1e6 if t > 0 else None,
@@ -382,7 +436,7 @@ def encoder_setup(args, device, rank: int, world: int):
     return model, batches_of, (lo, hi)
 
 
-def encoder_bench(args, device, steps=3, warmup=2):
+def encoder_bench(args, device):
     """Device-resident timing of the forward at the reference's batch size (64, `per_gpu_batch_size`) and at the
     grouped batch this framework uses (`encode_group`)."""
     model, batches_of, _ = encoder_setup(args, device, 0, 1)
@@ -394,19 +448,19 @@ def encoder_bench(args, device, steps=3, warmup=2):
         def run():
             return torch.cat([model.forward_varlen(ids, cu, mx, None, T) for ids, cu, mx, T in batches], 0)
 
-        for _ in range(warmup):
+        for _ in range(args.warmup):
             run()
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         sampler = ClockSampler(device.index or 0)
         sampler.start()
         e0.record()
-        for _ in range(steps):
+        for _ in range(args.steps):
             run()
         e1.record()
         torch.cuda.synchronize()
         clocks = sampler.stop()
-        ms = e0.elapsed_time(e1) / steps
+        ms = e0.elapsed_time(e1) / args.steps
         flops = 169.9e6 * total_tokens
         out[f"batch_{bs}"] = {"queries": args.nq, "tokens": total_tokens, "ms": ms, "queries_per_s": args.nq / ms * 1e3,
                               "gemm_tflops": flops / ms / 1e9, "launches": model.launches * len(batches), "clocks": clocks}
@@ -656,6 +710,27 @@ def scan_source_hash() -> str:
     return h.hexdigest()[:16]
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, I: torch.Tensor, D: torch.Tensor, limit: int = DUMP_LIMIT_BYTES) -> dict:
+    """Writes what a caller of the timed search received: ids as float64 (exact below 2**53) and scores as float32.
+    When both together would pass `limit` bytes, the same rows of each are written for a sample of queries drawn with
+    a fixed seed, and the row numbers go to rows.npy, so runs with the same arguments always write the same rows."""
+    ids = I.cpu().numpy().astype(np.float64)
+    scores = D.cpu().numpy().astype(np.float32)
+    arrays = {"ids": ids, "scores": scores}
+    nq = ids.shape[0]
+    max_rows = (limit - 4096) // (ids.shape[1] * (8 + 4) + 8)     # 4 KB leaves room for the three .npy headers
+    if nq > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(nq, max_rows, replace=False))
+        arrays = {"ids": ids[rows], "scores": scores[rows], "rows": rows.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name: list(a.shape) for name, a in arrays.items()}
+
+
 def workload_name(args):
     return (f"IVF-PQ nlist={args.nlist} M={args.m} nbits=8 nprobe={args.nprobe}, {args.n}x{args.d} synthetic gmm, "
             f"top-k={args.k}, batch of {args.nq} queries")
@@ -672,6 +747,7 @@ def make_config(args, world):
 
 # ----------------------------------------------------------------------------------------------------------
 def main():
+    sys.dont_write_bytecode = True   # the tree may be read-only: the project modules imported below leave no __pycache__
     args = parse()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -922,7 +998,7 @@ def main():
         extra["recall"] = recall_block(I_keep[:n_gt], gt_I, args.k)
         log("recall:", extra["recall"])
     if not args.no_encoder:
-        c5 = c5_encode_plus_search(args, device, rank, world, searcher, xq, steps=max(2, min(5, args.steps)), warmup=2)
+        c5 = c5_encode_plus_search(args, device, rank, world, searcher, xq, steps=args.steps, warmup=args.warmup)
         if rank == 0:
             extra["c5_encode_plus_search"] = c5
             if "recall" in extra:
@@ -988,6 +1064,8 @@ def main():
         if ranks_out is not None:
             out["per_rank"] = ranks_out
         out.update(extra)
+        if args.dump_outputs:
+            log(f"outputs of the last timed step -> {args.dump_outputs}:", dump_outputs(args.dump_outputs, I_keep, D_keep))
         print(json.dumps(out), flush=True)
     if world > 1:
         torch.distributed.barrier()
