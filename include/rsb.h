@@ -219,8 +219,21 @@ int rsb_bert_forward(rsb_bert_t* h, const int32_t* input_ids_dev, const int32_t*
                      const int32_t* cu_seqlens_dev, int B, int T, int max_seqlen, int pooling, void* out_f16_dev,
                      void* ws_dev, size_t ws_bytes, rsb_stream_t stream);
 int64_t rsb_bert_launches(rsb_bert_t* h);
+/* the forward's attention on its own: softmax(Q K^T / 8) V per (sequence, head) of the un-padded qkv_f16_dev
+ * [T, 3 x 768] (Q | K | V of each token, heads of 64 contiguous) into ctx_f16_dev [T, 768]; cu_seqlens_dev [B+1] int32,
+ * max_seqlen >= the longest sequence (<= 512) */
+int rsb_bert_attention(rsb_bert_t* h, const void* qkv_f16_dev, const int32_t* cu_seqlens_dev, int B, int T, int max_seqlen,
+                       void* ctx_f16_dev, rsb_stream_t stream);
+/* the forward's LayerNorm on its own (eps of the handle): in / out [T, 768], gamma / beta [768], all fp16 */
+int rsb_bert_layernorm(rsb_bert_t* h, const void* in_f16_dev, int T, const void* gamma_f16_dev, const void* beta_f16_dev,
+                       void* out_f16_dev, rsb_stream_t stream);
 /* the encoder's tensor-core GEMM on its own: C[M,N] = A[M,K] . W[N,K]^T + bias (epilogue 0), GELU (1) or
- * + residual (2); all fp16 row-major device pointers, N % 128 == 0, K % 64 == 0 */
+ * + residual (2); all fp16 row-major device pointers, N % 128 == 0, K % 64 == 0.  N % 256 == 0 up to 4096 runs the
+ * CTA-pair kernel the forward uses, other N a one-tile-per-CTA kernel.  `epilogue | RSB_GEMM_ROWS_REVERSED` makes the
+ * CTA-pair kernel visit the row tiles last-to-first (the order of the forward's FFN2); the one-tile-per-CTA kernel has
+ * no tile order and ignores it, and so does every call when the environment sets RSB_NO_SNAKE.  The result is the same
+ * either way. */
+#define RSB_GEMM_ROWS_REVERSED 0x100
 int rsb_gemm_f16(const void* A_dev, const void* W_dev, const void* bias_dev, const void* residual_dev, void* C_dev,
                  int M, int N, int K, int epilogue, rsb_stream_t stream);
 

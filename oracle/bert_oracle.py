@@ -82,3 +82,54 @@ def bert_forward(sd: Dict[str, torch.Tensor], config: dict, input_ids, attention
     if pooling == "average":
         return last.sum(dim=1) / attention_mask.sum(dim=1)[..., None].to(dtype)   # contriever.py:49
     return last[:, 0]                                        # contriever.py:51
+
+
+# ---- float64 references of the single encoder kernels, computed from the fp16 tensors the kernel receives ----------
+
+def gemm_f64(A, W, bias, residual=None, gelu=False):
+    """(A W^T + bias, then erf GELU or + residual) in float64, and |A| |W|^T (the scale of the accumulation error).
+    The dense part is returned too: the kernel rounds it to fp16 before it adds the residual."""
+    A64, W64 = A.double(), W.double()
+    dense = A64 @ W64.T + bias.double()
+    absprod = A64.abs() @ W64.abs().T
+    if gelu:
+        out = 0.5 * dense * (1.0 + torch.erf(dense / math.sqrt(2.0)))
+    elif residual is not None:
+        out = dense + residual.double()
+    else:
+        out = dense
+    return out, dense, absprod
+
+
+def attention_f64(qkv, cu_seqlens, heads: int = 12, head_dim: int = 64, scale: float = 0.125):
+    """softmax(Q K^T scale) V per (sequence, head) over the un-padded qkv [T, 3 * heads * head_dim] (Q | K | V of each
+    token).  Returns ctx [T, heads * head_dim] and sum_j p_j |v_j| [T, heads * head_dim], both float64."""
+    H = heads * head_dim
+    x = qkv.double()
+    T = x.shape[0]
+    ctx = torch.zeros((T, H), dtype=torch.float64, device=x.device)
+    pv_abs = torch.zeros_like(ctx)
+    cu = [int(c) for c in cu_seqlens]
+    lens = [cu[i + 1] - cu[i] for i in range(len(cu) - 1)]
+    # sequences of equal length are batched together
+    for S in sorted(set(lens)):
+        if S == 0:
+            continue
+        starts = torch.tensor([cu[i] for i, n in enumerate(lens) if n == S], device=x.device)
+        rows = (starts[:, None] + torch.arange(S, device=x.device)[None]).reshape(-1)
+        blk = x[rows].view(-1, S, 3, heads, head_dim).permute(2, 0, 3, 1, 4)   # [3, nseq, heads, S, hd]
+        q, k, v = blk[0], blk[1], blk[2]
+        p = torch.softmax((q @ k.transpose(-1, -2)) * scale, dim=-1)
+        ctx[rows] = (p @ v).permute(0, 2, 1, 3).reshape(-1, H)
+        pv_abs[rows] = (p @ v.abs()).permute(0, 2, 1, 3).reshape(-1, H)
+    return ctx, pv_abs
+
+
+def layernorm_f64(x, gamma, beta, eps: float):
+    """Row LayerNorm (biased variance) in float64.  Returns the output, 1 / sqrt(var + eps) and mean |x| per row."""
+    x64 = x.double()
+    mean = x64.mean(dim=1, keepdim=True)
+    var = ((x64 - mean) ** 2).mean(dim=1, keepdim=True)
+    rstd = 1.0 / torch.sqrt(var + eps)
+    out = (x64 - mean) * rstd * gamma.double() + beta.double()
+    return out, rstd, x64.abs().mean(dim=1, keepdim=True)

@@ -13,6 +13,7 @@ LIB_PATH = os.environ.get("RSB_LIBRARY") or os.path.join(_HERE, "librsb.so")
 RSB_OK = 0
 RSB_ERR_INVALID, RSB_ERR_CUDA, RSB_ERR_STATE, RSB_ERR_UNSUPPORTED, RSB_ERR_OOM = -1, -2, -3, -4, -5
 RSB_FLAT, RSB_IVFFLAT, RSB_IVFPQ = 0, 1, 2
+RSB_GEMM_ROWS_REVERSED = 0x100      # rsb_gemm_f16 epilogue flag
 (INFO_KIND, INFO_D, INFO_NLIST, INFO_M, INFO_NBITS, INFO_NTOTAL, INFO_IS_TRAINED, INFO_MAX_LIST_LEN,
  INFO_INDEX_BYTES) = range(9)
 PROF_NAMES = ("coarse_ms", "setup_ms", "lut_ms", "scan_ms", "merge_ms", "scan_bytes", "pairs", "launches", "scan_path")
@@ -67,6 +68,8 @@ SIGNATURES = [
     ("rsb_bert_forward", c_int, [_H, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                  c_size_t, c_void_p]),
     ("rsb_bert_launches", c_int64, [_H]),
+    ("rsb_bert_attention", c_int, [_H, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    ("rsb_bert_layernorm", c_int, [_H, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p]),
     ("rsb_gemm_f16", c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     ("rsb_debug_smem_base", c_int, []),
     ("rsb_pq_layout_offset", c_int, [c_int, c_int, c_int]),

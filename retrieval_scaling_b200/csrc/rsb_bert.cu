@@ -533,7 +533,10 @@ __device__ __forceinline__ void warp_layernorm_store(float (&x)[24], const __hal
 #pragma unroll
     for (int i = 0; i < 24; ++i) s += x[i];
     for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    const float mean = s * (1.f / HID);
+    // __fmul_rn: the mean is rounded before it is subtracted.  A plain multiply was contracted into x - s * (1/768) as
+    // one FFMA, which for a constant row (s = 768 x exactly) leaves -x * 2^-25 instead of 0.  Next to eps = 1e-12 that
+    // residue is not small: the row came out as up to beta -+ gamma instead of beta.
+    const float mean = __fmul_rn(s, 1.f / HID);
     float v = 0.f;
 #pragma unroll
     for (int i = 0; i < 24; ++i) { const float dlt = x[i] - mean; v = fmaf(dlt, dlt, v); }
@@ -644,7 +647,7 @@ void layernorm_rows_kernel(const __half* __restrict__ in, int T, const __half* _
 #pragma unroll
         for (int i = 0; i < 24; ++i) s += x[i];
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        const float mean = s * (1.f / HID);
+        const float mean = __fmul_rn(s, 1.f / HID);     // rounded before the subtraction, as in warp_layernorm_store
         float v = 0.f;
 #pragma unroll
         for (int i = 0; i < 24; ++i) { const float dlt = x[i] - mean; v = fmaf(dlt, dlt, v); }
@@ -1137,6 +1140,67 @@ int launch_gemm(const __half* A, int M, const Linear& lin, __half* C, const __ha
     return RSB_OK;
 }
 
+// LayerNorm over 768 of T rows (one launch), shared by the forward and rsb_bert_layernorm
+void launch_layernorm(const rsb_bert* h, const __half* x, int T, const __half* g, const __half* b, __half* out, cudaStream_t st) {
+    static const bool ln_v1 = getenv("RSB_LN_V1") != nullptr;
+    const int rows_per_block = 8;   // 256 threads = 8 warps = 8 rows
+    const int ln_grid = (T + rows_per_block - 1) / rows_per_block;
+    const int ln_rows_grid = std::min(ln_grid, 3 * rsb::device_num_sms());   // 24 warps per SM, ~12 rows per warp at 41k tokens
+    if (ln_v1) layernorm_kernel<<<ln_grid, 256, 0, st>>>(x, T, g, b, h->eps, out);
+    else layernorm_rows_kernel<<<ln_rows_grid, 256, 0, st>>>(x, T, g, b, h->eps, out);
+}
+
+// The list of sequences longer than 32 tokens that the flash kernel takes, written once per forward (one launch when
+// max_seqlen > 32, none otherwise; the count of launches is returned through *launches).
+int prepare_attention(rsb_bert* h, const int* cu_seqlens, int B, int max_seqlen, cudaStream_t st, long* launches) {
+    static rsb::PerDeviceFlag att_configured;
+    if (att_configured.first())
+        cudaFuncSetAttribute(attention_mma32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * ATT32_WARP_BYTES);
+    if (!h->side) {
+        cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking);
+        cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
+        cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
+    }
+    if (max_seqlen <= 32) return RSB_OK;
+    if (h->long_cap < B) {
+        cudaFree(h->long_list);
+        h->long_list = nullptr;
+        h->long_cap = 0;
+        if (cudaMalloc(&h->long_list, ((size_t)B + 1) * sizeof(int)) != cudaSuccess) return RSB_ERR_OOM;
+        h->long_cap = B;
+    }
+    cudaMemsetAsync(h->long_list + h->long_cap, 0, sizeof(int), st);          // the count lives behind the list
+    collect_long_kernel<<<(B + 255) / 256, 256, 0, st>>>(cu_seqlens, B, 32, h->long_list, h->long_list + h->long_cap);
+    ++*launches;
+    return RSB_OK;
+}
+
+// softmax(Q K^T / 8) V of every (sequence, head) of the un-padded [T, 3 x 768] QKV into ctx [T, 768] (after
+// prepare_attention for the same cu_seqlens / max_seqlen).  Sequences of <= 32 tokens (queries): warp-per-(sequence,
+// head) tensor-core kernel; longer ones (passages, the odd long query): flash-style kernel on a side stream -- the two
+// work on disjoint sequences of the same buffers.
+void launch_attention(rsb_bert* h, const __half* qkv, const int* cu_seqlens, int B, int max_seqlen, __half* ctx,
+                      cudaStream_t st, long* launches) {
+    const bool have_long = max_seqlen > 32;
+    if (have_long) {
+        cudaEventRecord(h->ev_fork, st);
+        cudaStreamWaitEvent(h->side, h->ev_fork, 0);
+        const int nqb = (max_seqlen + 127) / 128;
+        const long items = (long)B * h->heads * nqb;
+        const int fgrid = (int)std::min<long>(items, 2L * rsb::device_num_sms());   // 194 registers: two resident blocks per SM
+        attention_flash_kernel<<<fgrid, 128, 0, h->side>>>(qkv, cu_seqlens, ctx, 0.125f, h->long_list, h->long_list + h->long_cap,
+                                                           h->heads, nqb);
+        cudaEventRecord(h->ev_join, h->side);
+        ++*launches;
+    }
+    const int nwarps = B * h->heads;
+    static const bool no_snake = getenv("RSB_NO_SNAKE") != nullptr;
+    attention_mma32_kernel<<<(nwarps + 3) / 4, 128, 4 * ATT32_WARP_BYTES, st>>>(qkv, cu_seqlens, ctx, 0.125f, h->heads, B,
+                                                                               no_snake ? 0 : 1);
+    ++*launches;
+    if (have_long) cudaStreamWaitEvent(st, h->ev_join, 0);   // join before the attention-output GEMM
+}
+
 }  // namespace
 
 extern "C" const char* rsb_bert_last_error(void) { return g_berr.c_str(); }
@@ -1274,54 +1338,7 @@ extern "C" int rsb_bert_forward(rsb_bert_t* h, const int32_t* input_ids, const i
     embed_ln_kernel<<<ln_grid, 256, 0, st>>>(input_ids, token_type_ids, cu_seqlens, B, T, h->word, h->pos, h->type,
                                              h->emb_g, h->emb_b, h->eps, h->vocab, h->max_pos, Hs);
     h->launches++;
-    static rsb::PerDeviceFlag att_configured;
-    if (att_configured.first())
-        cudaFuncSetAttribute(attention_mma32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 4 * ATT32_WARP_BYTES);
-    if (!h->side) {
-        cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking);
-        cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
-        cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
-    }
-    const bool have_long = max_seqlen > 32;
-    if (have_long) {                                     // list of the sequences the flash kernel has to take, once per forward
-        if (h->long_cap < B) {
-            cudaFree(h->long_list);
-            h->long_list = nullptr;
-            h->long_cap = 0;
-            if (cudaMalloc(&h->long_list, ((size_t)B + 1) * sizeof(int)) != cudaSuccess) return bfail(RSB_ERR_OOM, "long-sequence list");
-            h->long_cap = B;
-        }
-        cudaMemsetAsync(h->long_list + h->long_cap, 0, sizeof(int), st);          // the count lives behind the list
-        collect_long_kernel<<<(B + 255) / 256, 256, 0, st>>>(cu_seqlens, B, 32, h->long_list, h->long_list + h->long_cap);
-        h->launches++;
-    }
-    static const bool ln_v1 = getenv("RSB_LN_V1") != nullptr;
-    const int ln_rows_grid = std::min(ln_grid, 3 * rsb::device_num_sms());   // 24 warps per SM, ~12 rows per warp at 41k tokens
-    auto launch_ln = [&](const __half* x, const __half* g, const __half* b) {
-        if (ln_v1) layernorm_kernel<<<ln_grid, 256, 0, st>>>(x, T, g, b, h->eps, Hs);
-        else layernorm_rows_kernel<<<ln_rows_grid, 256, 0, st>>>(x, T, g, b, h->eps, Hs);
-    };
-    auto launch_attention = [&](const __half* qkv_p, __half* ctx_p) {
-        // sequences of <= 32 tokens (queries): warp-per-(sequence, head) tensor-core kernel; longer ones (passages, the odd
-        // long query): flash-style kernel on a side stream -- the two work on disjoint sequences of the same buffers
-        if (have_long) {
-            cudaEventRecord(h->ev_fork, st);
-            cudaStreamWaitEvent(h->side, h->ev_fork, 0);
-            const int nqb = (max_seqlen + 127) / 128;
-            const long items = (long)B * h->heads * nqb;
-            const int fgrid = (int)std::min<long>(items, 2L * rsb::device_num_sms());   // 194 registers: two resident blocks per SM
-            attention_flash_kernel<<<fgrid, 128, 0, h->side>>>(qkv_p, cu_seqlens, ctx_p, 0.125f, h->long_list, h->long_list + h->long_cap,
-                                                               h->heads, nqb);
-            cudaEventRecord(h->ev_join, h->side);
-            h->launches++;
-        }
-        const int nwarps = B * h->heads;
-        static const bool no_snake = getenv("RSB_NO_SNAKE") != nullptr;
-        attention_mma32_kernel<<<(nwarps + 3) / 4, 128, 4 * ATT32_WARP_BYTES, st>>>(qkv_p, cu_seqlens, ctx_p, 0.125f, h->heads, B,
-                                                                                   no_snake ? 0 : 1);
-        h->launches++;
-        if (have_long) cudaStreamWaitEvent(st, h->ev_join, 0);   // join before the attention-output GEMM
-    };
+    if (prepare_attention(h, cu_seqlens, B, max_seqlen, st, &h->launches) != RSB_OK) return bfail(RSB_ERR_OOM, "long-sequence list");
     // RSB_BERT_PROFILE=1 (diagnostic): CUDA events between the kernels of the forward, summed per kernel kind over the
     // layers and printed to stderr after each forward -- per-kernel times INSIDE a back-to-back run (ncu's are isolated,
     // cold-cache and at other clocks).  Synchronises the stream; never set in a timed run.
@@ -1340,17 +1357,17 @@ extern "C" int rsb_bert_forward(rsb_bert_t* h, const int32_t* input_ids, const i
         Layer& l = h->L[li];
         if (launch_gemm<EPI_BIAS>(Hs, T, l.qkv, QKV, nullptr, st) != RSB_OK) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
         mark();
-        launch_attention(QKV, CTX);
+        launch_attention(h, QKV, cu_seqlens, B, max_seqlen, CTX, st, &h->launches);
         mark();
         if (launch_gemm<EPI_BIAS_RESIDUAL>(CTX, T, l.attn_out, TMP, Hs, st) != RSB_OK) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
         mark();
-        launch_ln(TMP, l.ln1_g, l.ln1_b);
+        launch_layernorm(h, TMP, T, l.ln1_g, l.ln1_b, Hs, st);
         mark();
         if (launch_gemm<EPI_BIAS_GELU>(Hs, T, l.ffn1, FF, nullptr, st) != RSB_OK) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
         mark();
         if (launch_gemm<EPI_BIAS_RESIDUAL>(FF, T, l.ffn2, TMP, Hs, st, true) != RSB_OK) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
         mark();
-        launch_ln(TMP, l.ln2_g, l.ln2_b);
+        launch_layernorm(h, TMP, T, l.ln2_g, l.ln2_b, Hs, st);
         mark();
         h->launches += 6;   // + the attention launch(es), counted in launch_attention
     }
@@ -1377,21 +1394,53 @@ extern "C" int rsb_bert_forward(rsb_bert_t* h, const int32_t* input_ids, const i
 
 extern "C" int64_t rsb_bert_launches(rsb_bert_t* h) { return h ? h->launches : 0; }
 
-// plain GEMM entry (tests / roofline of the tensor-core kernel): C[M,N] = A[M,K] W[N,K]^T + bias, epilogue as above
+// the forward's attention on its own: qkv [T, 3 x 768] (Q | K | V per token), ctx [T, 768], all fp16
+extern "C" int rsb_bert_attention(rsb_bert_t* h, const void* qkv_f16, const int32_t* cu_seqlens, int B, int T, int max_seqlen,
+                                  void* ctx_f16, rsb_stream_t stream) {
+    if (!h || !qkv_f16 || !cu_seqlens || !ctx_f16) return bfail(RSB_ERR_INVALID, "null argument");
+    if (B <= 0 || T <= 0) return bfail(RSB_ERR_INVALID, "empty batch");
+    if (max_seqlen > ATT_MAXS) return bfail(RSB_ERR_UNSUPPORTED, "sequence longer than %s%ld tokens", "", (long)ATT_MAXS);
+    cudaStream_t st = (cudaStream_t)stream;
+    long launches = 0;
+    if (prepare_attention(h, cu_seqlens, B, max_seqlen, st, &launches) != RSB_OK) return bfail(RSB_ERR_OOM, "long-sequence list");
+    launch_attention(h, static_cast<const __half*>(qkv_f16), cu_seqlens, B, max_seqlen, static_cast<__half*>(ctx_f16), st, &launches);
+    cudaError_t e = cudaPeekAtLastError();
+    if (e != cudaSuccess) return bfail(RSB_ERR_CUDA, "attention launch failed: %s", cudaGetErrorString(e));
+    return RSB_OK;
+}
+
+// the forward's LayerNorm on its own (eps of the handle): in / out [T, 768], gamma / beta [768], all fp16
+extern "C" int rsb_bert_layernorm(rsb_bert_t* h, const void* in_f16, int T, const void* gamma, const void* beta, void* out_f16,
+                                  rsb_stream_t stream) {
+    if (!h || !in_f16 || !gamma || !beta || !out_f16) return bfail(RSB_ERR_INVALID, "null argument");
+    if (T <= 0) return bfail(RSB_ERR_INVALID, "empty batch");
+    launch_layernorm(h, static_cast<const __half*>(in_f16), T, static_cast<const __half*>(gamma), static_cast<const __half*>(beta),
+                     static_cast<__half*>(out_f16), (cudaStream_t)stream);
+    cudaError_t e = cudaPeekAtLastError();
+    if (e != cudaSuccess) return bfail(RSB_ERR_CUDA, "layernorm launch failed: %s", cudaGetErrorString(e));
+    return RSB_OK;
+}
+
+// plain GEMM entry (tests / roofline of the tensor-core kernel): C[M,N] = A[M,K] W[N,K]^T + bias, epilogue as above;
+// RSB_GEMM_ROWS_REVERSED in `epilogue` visits the row tiles last-to-first, as FFN2 does inside the forward
 extern "C" int rsb_gemm_f16(const void* A, const void* W, const void* bias, const void* residual, void* C, int M, int N,
                             int K, int epilogue, rsb_stream_t stream) {
     if (!A || !W || !bias || !C) return bfail(RSB_ERR_INVALID, "null argument");
     if (M <= 0 || N % G_BN || K % G_BK || N <= 0 || K <= 0) return bfail(RSB_ERR_INVALID, "need N %% 128 == 0 and K %% 64 == 0");
+    const bool m_rev = (epilogue & RSB_GEMM_ROWS_REVERSED) != 0;
+    epilogue &= ~RSB_GEMM_ROWS_REVERSED;
     if (epilogue == EPI_BIAS_RESIDUAL && !residual) return bfail(RSB_ERR_INVALID, "residual is NULL");
     Linear lin;
     lin.w = (__half*)W; lin.b = (__half*)bias; lin.N = N; lin.K = K;
-    if (!make_map(&lin.map, W, N, K, G_BN)) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
+    lin.map_ok = make_map(&lin.map, W, N, K, G_BN);      // launch_gemm takes the pair kernel only with a valid map
+    if (!lin.map_ok) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
     lin.pair_ok = (N % H_BN == 0) && N <= H_BIAS_MAX;
     cudaStream_t st = (cudaStream_t)stream;
+    const __half* Ah = (const __half*)A;
     int rc;
-    if (epilogue == EPI_BIAS) rc = launch_gemm<EPI_BIAS>((const __half*)A, M, lin, (__half*)C, nullptr, st);
-    else if (epilogue == EPI_BIAS_GELU) rc = launch_gemm<EPI_BIAS_GELU>((const __half*)A, M, lin, (__half*)C, nullptr, st);
-    else if (epilogue == EPI_BIAS_RESIDUAL) rc = launch_gemm<EPI_BIAS_RESIDUAL>((const __half*)A, M, lin, (__half*)C, (const __half*)residual, st);
+    if (epilogue == EPI_BIAS) rc = launch_gemm<EPI_BIAS>(Ah, M, lin, (__half*)C, nullptr, st, m_rev);
+    else if (epilogue == EPI_BIAS_GELU) rc = launch_gemm<EPI_BIAS_GELU>(Ah, M, lin, (__half*)C, nullptr, st, m_rev);
+    else if (epilogue == EPI_BIAS_RESIDUAL) rc = launch_gemm<EPI_BIAS_RESIDUAL>(Ah, M, lin, (__half*)C, (const __half*)residual, st, m_rev);
     else return bfail(RSB_ERR_INVALID, "unknown epilogue");
     if (rc != RSB_OK) return bfail(RSB_ERR_CUDA, "tensor map encode failed");
     cudaError_t e = cudaPeekAtLastError();
